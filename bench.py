@@ -25,6 +25,8 @@ e2e    : same metric through the host-buffer C-ABI call: pinned host input -> H2
          (not page-locked) memory.  pcie: plain cudaMemcpy H2D / D2H peaks measured in the same run.
 --impl reference : the CPU path (oracle port of the reference; Nim is not available, so the
          reference itself cannot be built -- see DESIGN.md) on all host cores, bounded sample.
+--dump-outputs DIR : after the timed steps, write what the selected workload's timed path returned in its
+         last step as DIR/<name>.npy (see dump_members), so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -46,6 +48,7 @@ BLOCKS_PER_GPU = 65536
 C5_BLOCKS_PER_GPU = 131072
 C3_MEMBERS = 65536
 C4_TILES = 6118
+DUMP_LIMIT = 64 * 10 ** 6   # bytes: every file --dump-outputs writes in one run, all ranks together
 PUBLISHED_C1 = {"uncompress_alice29_ms": 0.233, "compress_best_speed_alice29_ms": 0.643,
                 "hardware": "Ryzen 5 5600X, 1 thread (README.md:41,63); different machine"}
 
@@ -559,6 +562,11 @@ def measure_compress(e, d_src, src_offs, level, steps, warmup, n_total_members, 
         launches[0] += tm["kernel_launches"]
 
     ms = timed(e, step_timed, steps)
+    if e.dump_dir:   # here, before the e2e legs: c5's writes d_dst again through the host-input call
+        from zippy_b200 import _native
+        sizes, inv = np.unique(np.diff(src_offs), return_inverse=True)
+        bound = np.array([_native.lib().zb200_compress_bound(int(s), z.dfGzip) for s in sizes], dtype=np.uint64)
+        dump_members(e, d_dst, state["oo"], bound[inv])
     res["clocks"] = e.last_clocks
     res["ms_per_step"] = ms
     res["value"] = e.world * in_bytes / GIB / (ms / 1e3)   # weak scaling: every rank has in_bytes
@@ -736,6 +744,7 @@ def measure_uncompress(e, d_comp, comp_offs, out_sizes, steps, warmup, do_e2e=Tr
         acc["inflate_ms"] += tm["inflate_ms"]
         acc["verify_ms"] += tm["verify_ms"]
         acc["launches"] += tm["kernel_launches"]
+        acc["last"] = (lens, st)
         return lens, st
 
     for _ in range(max(1, warmup)):
@@ -746,7 +755,8 @@ def measure_uncompress(e, d_comp, comp_offs, out_sizes, steps, warmup, do_e2e=Tr
     per = {"inflate_ms": acc["inflate_ms"] / steps, "verify_ms": acc["verify_ms"] / steps}
     res = {"clocks": e.last_clocks, "ms_per_step": ms, "in_bytes": in_bytes, "out_bytes": out_bytes, "in_gibs": in_bytes / GIB / (ms / 1e3),
            "out_gibs": out_bytes / GIB / (ms / 1e3), "gpu_launches": acc["launches"],
-           "roofline": roofline(e, "k_inflate", per["inflate_ms"], in_bytes + out_bytes, per), "_d_out": d_out, "_doffs": doffs}
+           "roofline": roofline(e, "k_inflate", per["inflate_ms"], in_bytes + out_bytes, per), "_d_out": d_out, "_doffs": doffs,
+           "_lens": acc["last"][0], "_st": acc["last"][1]}
     if do_e2e:
         from zippy_b200 import _native
         L = _native.lib()
@@ -823,6 +833,36 @@ def strip(d):
     return {k: v for k, v in d.items() if not k.startswith("_")}
 
 
+def save_output(e, name, arr):
+    """DIR/<name>.npy (rank<r>_<name>.npy when several ranks each hold a shard)."""
+    os.makedirs(e.dump_dir, exist_ok=True)
+    prefix = "rank%d_" % e.rank if e.world > 1 else ""
+    np.save(os.path.join(e.dump_dir, prefix + name + ".npy"), arr)
+
+
+def dump_members(e, d_buf, offsets, max_bytes, **returned):
+    """--dump-outputs for a batch call: member i of the result lies in d_buf[offsets[i]:offsets[i + 1]].
+    Every member is covered by offsets.npy, crc32.npy and the call's other per-member results (`returned`),
+    all float64, which holds them exactly.  The CRC-32s come from the build's own checksum kernel: a
+    fingerprint of the bytes, not an independent check of them.  sample_bytes.npy holds the bytes (as
+    float32) of the whole members listed in sample_index.npy, concatenated in that order.  The sample is a
+    seeded draw over max_bytes, a bound of each member's size known before the call, so it does not depend
+    on what the build produced; it is sized so that the files of all ranks together stay within DUMP_LIMIT."""
+    n = len(offsets) - 1
+    crc = e.ctx.checksum_batch_device(d_buf.data_ptr(), offsets, "crc32")
+    full = dict(offsets=offsets, crc32=crc, **returned)
+    budget = DUMP_LIMIT // e.world - sum(8 * len(a) + 256 for a in full.values()) - 2 * 256   # 256: .npy header
+    assert budget >= 0, "too many members per rank for a %d-byte dump" % DUMP_LIMIT
+    order = np.random.default_rng(0).permutation(n)
+    cost = 4 * max_bytes[order].astype(np.int64) + 8   # float32 bytes + a float64 index
+    idx = np.sort(order[:np.searchsorted(np.cumsum(cost), budget, side="right")])
+    sample = e.torch.cat([d_buf[int(offsets[i]):int(offsets[i + 1])] for i in idx]) if len(idx) else d_buf[:0]
+    for name, a in full.items():
+        save_output(e, name, a.astype(np.float64))
+    save_output(e, "sample_index", idx.astype(np.float64))
+    save_output(e, "sample_bytes", sample.cpu().numpy().astype(np.float32))
+
+
 # -------------------------------------------------------------------------------------
 # the five workloads
 # -------------------------------------------------------------------------------------
@@ -870,7 +910,7 @@ def run_c2(e, args, steps, warmup, full=True):
     return out
 
 
-def run_c1(e, args, reps=30):
+def run_c1(e, args, reps=30, warmup=1):
     """Config 1: one file through the drop-in calls; wall-clock latency of a synchronous call."""
     import zlib
     from oracle import oracle as o
@@ -879,12 +919,15 @@ def run_c1(e, args, reps=30):
     raw = util.load_corpus()["alice29.txt"]
     gold_gz = util.load_golden()["alice29.txt.gz"][0]
 
+    last = [None]   # what the last timed call returned
+
     def lat(f, k=reps):
-        f()
+        for _ in range(warmup):
+            f()
         ts = []
         for _ in range(k):
             t0 = time.perf_counter()
-            f()
+            last[0] = f()
             ts.append((time.perf_counter() - t0) * 1e3)
         return float(np.median(ts)), float(min(ts))
 
@@ -893,8 +936,13 @@ def run_c1(e, args, reps=30):
     assert z.uncompress(comp) == raw and z.uncompress(gold_gz) == raw   # round trip bit-exact + the reference's own .gz
     c_med, c_min = lat(lambda: z.compress(raw, z.BestSpeed, z.dfGzip))
     tm_c = e.z.default_context().timing()
+    if e.dump_dir:   # without the gzip header: its FNAME length is drawn at random on every call (zippy.nim:28-42)
+        body = last[0][last[0].index(0, 10) + 1:]
+        save_output(e, "compressed_after_header", np.frombuffer(body, dtype=np.uint8).astype(np.float32))
     u_med, u_min = lat(lambda: z.uncompress(gold_gz))
     tm_u = e.z.default_context().timing()
+    if e.dump_dir:
+        save_output(e, "uncompressed", np.frombuffer(last[0], dtype=np.uint8).astype(np.float32))
     oc_med, oc_min = lat(lambda: o.compress(raw, 1, o.dfGzip))
     ou_med, ou_min = lat(lambda: o.uncompress(gold_gz))
     zc_med, _ = lat(lambda: zlib.compress(raw, 1))
@@ -933,6 +981,9 @@ def run_c3(e, args, steps, warmup):
     sizes, st = ctx.uncompressed_sizes_device(d_src.data_ptr(), offs, z.dfDetect)
     assert not st.any()
     r = measure_uncompress(e, d_src, offs, sizes, steps, warmup, do_e2e=not args.no_e2e)
+    if e.dump_dir:
+        # offsets: the output slots passed in; lengths and status: what the last timed call returned
+        dump_members(e, r["_d_out"], r["_doffs"], sizes, lengths=r["_lens"], status=r["_st"])
     host = r["_d_out"][:int(r["_doffs"][23])].cpu().numpy()
     for i, nm in enumerate(names):   # byte-exact against the reference's fixtures (sha256 of the .gold / original)
         assert util.sha(host[int(r["_doffs"][i]):int(r["_doffs"][i + 1])].tobytes()) == golden[nm][1]["sha256"], nm
@@ -1144,16 +1195,17 @@ def run_reference(args, rank, world):
         raw = util.load_corpus()["alice29.txt"]
         gz = util.load_golden()["alice29.txt.gz"][0]
         ts = []
-        for _ in range(50):
+        for s in range(args.warmup + args.steps):
             t0 = time.perf_counter()
             c = o.compress(raw, 1, o.dfGzip)
             o.uncompress(gz)
-            ts.append((time.perf_counter() - t0) * 1e3)
+            if s >= args.warmup:
+                ts.append((time.perf_counter() - t0) * 1e3)
         val = float(np.median(ts))
         out = {"impl": "reference", "metric": "single_file_latency", "value": val, "unit": "ms", "n_gpus": args.gpus,
                "steps": args.steps, "warmup": args.warmup, "ms_per_step": val, "higher_is_better": False, "scaling": "weak",
                "vs_baseline": None, "dtype": "u8", "data": "synthetic", "config": {"workload": "C1: alice29.txt compress + uncompress"},
-               "cpu_baseline": {"value": val, "unit": "ms", "cores": 1, "kind": "port", "sample": "median of 50 calls"},
+               "cpu_baseline": {"value": val, "unit": "ms", "cores": 1, "kind": "port", "sample": "median of %d calls" % args.steps},
                "e2e": {"value": val, "unit": "ms", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
         print(json.dumps(out))
         return
@@ -1190,7 +1242,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="c2 only: skip the c1/c3/c4/c5 summaries")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--level", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed path's outputs of its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the GPU path's outputs (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -1205,10 +1262,12 @@ def main():
     clocks.mark()
     e.clocks = clocks
     e.last_clocks = None
+    e.dump_dir = args.dump_outputs   # the selected workload's outputs only, not the extras'
     w = args.workload
     extras = {}
     if w == "c2":
         out = run_c2(e, args, args.steps, args.warmup)
+        e.dump_dir = None
         main_clk = out.pop("clocks")
         if not args.no_extras:
             xs = max(2, min(args.steps, 3))
@@ -1228,7 +1287,7 @@ def main():
                 e.torch.cuda.empty_cache()
                 extras["c5"] = strip(run_c5(e, args, xs, 3))
     else:
-        fn = {"c1": lambda: run_c1(e, args), "c3": lambda: run_c3(e, args, args.steps, args.warmup),
+        fn = {"c1": lambda: run_c1(e, args, args.steps, args.warmup), "c3": lambda: run_c3(e, args, args.steps, args.warmup),
               "c4": lambda: run_c4(e, args, args.steps, args.warmup), "c5": lambda: run_c5(e, args, args.steps, args.warmup)}[w]
         out = fn()
         out.setdefault("scaling", "weak")
